@@ -33,6 +33,12 @@ N > 1 (torchrun): one rank per GPU, each probes its own device (weak scaling,
 no data-path collective) and the 512-byte result structs are all-gathered over
 NCCL — the one exchange step the path has; then rank 0 alone runs the
 single-process legs while the other ranks wait on a CPU (gloo) barrier.
+
+--dump-outputs DIR writes what the last probe of the `value` loop handed its
+caller (the device-written verdict and checksums) and a fixed sample of the
+region it left in HBM, as DIR/<name>.npy.  The pattern seed does not depend on
+which GPU of the box the run lands on, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,9 +55,14 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is cached beside the sources
 
 SWEEP_BYTES = 4 << 30
 READ_SWEEPS = COPY_SWEEPS = 5
+# The library seeds a device's pattern with seed_base | device minor; with the low 16 bits set the minor drops out, so
+# the bytes a run probes do not depend on which GPU it was given.  Ranks are kept apart above those bits.
+SEED_BASE = 0x00C0FFEE0000FFFF
+DUMP_BLOCKS, DUMP_BLOCK_WORDS = 64, 1024     # region sample: 64 seeded blocks of 1024 words (1 MiB as float64 halves)
 METRIC = "composed-GPU probes/sec"
 UNIT = "probes/s"
 WORKLOAD = "configs[1]: 1xB200 attach — HBM probe (fill + 5 read + 5 copy sweeps, S=4 GiB) + CDI/status JSON emit"
@@ -494,6 +505,26 @@ def churn_leg(cro, ctx, cycles, probe=True):
 # ---------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------
+def dump_outputs(out_dir, ctx, r, S):
+    """What the last timed probe computed, as float64 arrays; 64-bit words are split into exact (high, low) 32-bit halves.
+    The struct's times are left out: they are measurements, not results."""
+    import numpy as np
+
+    def halves(words):
+        w = np.asarray(words, dtype=np.uint64)
+        return np.stack([w >> np.uint64(32), w & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    # (checksum, closed form, copy checksum) x (xor, sum, position-weighted sum) x (high, low)
+    np.save(os.path.join(out_dir, "probe_checksums.npy"), halves([r.checksum, r.expect, r.copy_checksum]))
+    np.save(os.path.join(out_dir, "probe_seed.npy"), halves([r.seed]))
+    np.save(os.path.join(out_dir, "probe_verdict.npy"), np.array(
+        [r.status, r.fail_code, r.fail_index, r.copy_verified, r.read_sweeps, r.copy_sweeps, r.nonce, r.sweep_bytes], dtype=np.float64))
+    words = 2 * S // 8                     # both halves of the ping-pong region, as the last sweeps left them
+    n = min(DUMP_BLOCK_WORDS, words)
+    firsts = np.random.default_rng(0).integers(0, words - n + 1, DUMP_BLOCKS)
+    np.save(os.path.join(out_dir, "region_sample.npy"), halves([ctx.read_words(0, int(f), n) for f in firsts]))
+
+
 def run_ours(args, rank, local_rank, world):
     import torch
     cro = importlib.import_module("composable-resource-operator_b200")
@@ -513,7 +544,8 @@ def run_ours(args, rank, local_rank, world):
 
     t_init = time.perf_counter()
     ctx = cro.ProbeContext(sweep_bytes=S, devices=[local_rank], read_variant=args.read_variant,
-                           copy_variant=args.copy_variant, rank_base=rank, world=world, read_sweeps=READ_SWEEPS, copy_sweeps=COPY_SWEEPS)
+                           copy_variant=args.copy_variant, rank_base=rank, world=world, read_sweeps=READ_SWEEPS, copy_sweeps=COPY_SWEEPS,
+                           seed_base=SEED_BASE + (rank << 16))
     info = ctx.own_devices()[0]
     uuid = info.gpu_uuid.decode()
     ctx_create_s = time.perf_counter() - t_init
@@ -590,6 +622,8 @@ def run_ours(args, rank, local_rank, world):
         results.append(r)
     barrier()
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, results[-1], S)
 
     # ---- end to end through the reference-facing call: `e2e` ----------------
     barrier()
@@ -768,6 +802,7 @@ def main():
     ap.add_argument("--no-storm", action="store_true")
     ap.add_argument("--storm", type=int, default=1000)
     ap.add_argument("--cycles", type=int, default=100)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed probe computed as DIR/<name>.npy")
     args = ap.parse_args()
     # stdout must carry the ONE JSON line and nothing else, but libraries print there too (NCCL writes
     # "NCCL version ..." with printf at init).  Keep the real stdout aside and point fd 1 at stderr for
@@ -789,12 +824,7 @@ def main():
                 print("build_oracle() failed: %s" % e, file=sys.stderr)
         run_reference(args, rank, world)
         return
-    if rank == 0 or not os.path.exists(os.path.join(ROOT, "composable-resource-operator_b200", "libcroprobe.so")):
-        try:
-            g.build()
-        except Exception as e:   # the GPU box may lack nothing, but never hide a stale library behind a build error
-            print("build() failed: %s" % e, file=sys.stderr)
-    run_ours(args, rank, local_rank, world)
+    run_ours(args, rank, local_rank, world)     # runs what build() left in the tree; the import fails loudly without it
 
 
 if __name__ == "__main__":

@@ -345,6 +345,7 @@ int ctx_create(const cro_opts* o, cro_ctx** out) {
                 break;
             }
         }
+        for (const identity::ProcGpu& g : proc) c->proc_lists_mine = c->proc_lists_mine || g.uuid == uuid;
         keyed.push_back({std::move(d), key});
     }
     std::stable_sort(keyed.begin(), keyed.end(), [](const Keyed& a, const Keyed& b) { return a.key < b.key; });
@@ -1098,7 +1099,9 @@ int ctx_inventory(cro_ctx* c, std::vector<cro_dev_info>* out, bool force) {
     //   * in the BACKGROUND every 30 s — the reference's own requeue period (composableresource_controller.go:223,285)
     //     — because each such read goes through the driver's locks (100+ ms for a full box while nvidia-smi polls) and
     //     a reconcile must not pay for a refresh that will almost always confirm what is known.
-    std::string key = identity::ProcRegistryListing(c->proc_root);
+    // A registry that listed none of the devices CUDA had just opened describes some other view of the node (a container
+    // may mount it empty): it is not consulted, and the inventory goes by NVML as on a host without one.
+    std::string key = c->proc_lists_mine ? identity::ProcRegistryListing(c->proc_root) : std::string();
     const bool have_proc = !key.empty();
     if (!have_proc) key = "-";
     const auto now = std::chrono::steady_clock::now();

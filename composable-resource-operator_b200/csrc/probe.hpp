@@ -132,6 +132,7 @@ struct cro_ctx {
     bool peers_enabled = false;
     bool nvtx = true;
     std::string proc_root = "/proc";   // where the node's /proc is mounted (tests point it at a fake tree)
+    bool proc_lists_mine = false;      // at init the registry listed one of this context's devices (ctx_create)
     // the node's inventory as of the last enumeration (inventory.hpp)
     std::mutex inv_mu;
     std::string inv_key;               // uuid/minor set the cached list was built from

@@ -7,6 +7,7 @@ source and writes tests/golden/wire_structs.json.  Run from the repo root (needs
 No reference test reads a request body (SURVEY.md §8c: "parity unpinned" for the emitted bytes), so what CAN be pinned
 mechanically is pinned here: the names, the order and the omitempty flags encoding/json walks are the declarations'
 — tests/test_wire_structs.py holds the product's emitters and the oracle's type descriptions against them."""
+import hashlib
 import json
 import os
 import re
@@ -58,9 +59,12 @@ def extract():
 if __name__ == "__main__":
     got = extract()
     text = json.dumps(got, indent=1, sort_keys=True) + "\n"
+    # the seal tests/test_wire_structs.py holds the fixture to where the reference tree is not at hand
+    seal = hashlib.sha256(text.encode()).hexdigest() + "  wire_structs.json\n"
     if "--check" in sys.argv:
-        same = os.path.exists(OUT) and open(OUT).read() == text
+        same = all(os.path.exists(p) and open(p).read() == t for p, t in ((OUT, text), (OUT + ".sha256", seal)))
         print("wire_structs.json", "matches the reference" if same else "DIFFERS from the reference")
         sys.exit(0 if same else 1)
     open(OUT, "w").write(text)
+    open(OUT + ".sha256", "w").write(seal)
     print("wrote", sum(len(v) for v in got.values()), "structs from", len(got), "files")

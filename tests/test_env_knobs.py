@@ -7,11 +7,10 @@ import pytest
 REF_LINE = "the env variable DEVICE_RESOURCE_TYPE has an invalid value: '%s'"     # composableresource_adapter.go:44
 
 
-def test_wording_is_the_references(cro):
-    import os
-    ref = os.path.join("/root/reference", "internal", "controller", "composableresource_adapter.go")
-    if os.path.exists(ref):
-        assert REF_LINE in open(ref).read()
+def test_wording_is_the_references(cro, kats):
+    # the reference's own sentence, as its controller tests expect it (tests/golden/reference_kats.json "env_errors")
+    (ref,) = kats["env_errors"]
+    assert ref["error"] == REF_LINE % ref["device_resource_type"]
     msg = cro.validate_env("CRO_USE_GRAPH", "yes")
     assert msg == REF_LINE.replace("DEVICE_RESOURCE_TYPE", "CRO_USE_GRAPH") % "yes"
 

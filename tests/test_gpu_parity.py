@@ -282,9 +282,10 @@ def test_identity_strings_match_nvidia_smi(cro):
             alt = smi_csv("minor_number,gpu_uuid,pci.bus_id")
             if alt.returncode == 0:
                 assert cro.emit_csv(devs, "minor_number,gpu_uuid,pci.bus_id") == alt.stdout
-        # /proc flavour (gpus.go:1017-1037), when the driver exposes it in this container
+        # /proc flavour (gpus.go:1017-1037), when the driver exposes it in this container (a container may mount the
+        # registry empty; the enumeration above then came from NVML)
         base = "/proc/driver/nvidia/gpus"
-        if os.path.isdir(base):
+        if os.path.isdir(base) and os.listdir(base):
             lines = ""
             for name in sorted(os.listdir(base)):
                 p = os.path.join(base, name, "information")

@@ -41,8 +41,9 @@ def test_rke2_flavour_with_a_fake_proc(cro, tmp_path):
         out = cro.local_node_op(None, dict(req, op=op, proc_root=root))
         assert out["error"] == "" and [(x["kind"], x["how"]) for x in out["exec_log"]] == [("proc_scan", "native")], out
     # it is there: the next step needs nvidia-smi, which this container does not have — the spawn error is the exec error
+    # (native_nvml off: where libnvidia-ml is loadable the query would otherwise be answered in process)
     root = fake_proc(tmp_path / "b", {"0000:1f:00.0": ("0", DEV)})
-    out = cro.local_node_op(None, dict(req, op="drain", proc_root=root))
+    out = cro.local_node_op(None, dict(req, op="drain", proc_root=root, native_nvml=False))
     assert [(x["kind"], x["how"]) for x in out["exec_log"]] == [("proc_scan", "native"), ("command", "spawned")]
     assert out["exec_log"][1]["argv"] == ["/bin/chroot", "/host-root", "/usr/bin/nvidia-smi", "drain", "-p", "0000:1F:00.0", "-q"]
     if not os.path.exists("/usr/bin/nvidia-smi"):
